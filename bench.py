@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the vocoder hot path (contract: see the task statement / DESIGN.md "Measurement").
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl cube|reference] [--workload pwn|hifigan]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl cube|reference] [--workload pwn|hifigan] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic mel.  Default workload is
 BASELINE.json configs[1]: batch=8 x 10 s utterances, 80-bin synthetic mel, ParallelWaveNet (ClariNet
@@ -10,10 +10,13 @@ collective).  ``--workload hifigan`` runs configs[2] (batch=64 x 10 s, HiFi-GAN 
 
 Prints ONE JSON line (rank 0).  ``value`` is device-timed (CUDA events, inputs resident in HBM);
 ``e2e`` goes through the host-buffer C-ABI call with H2D/D2H inside the timed region.
+``--dump-outputs DIR`` writes what the timed path returned in its last timed step as DIR/<name>.npy (float32); the inputs
+are seeded, so two builds of the project can be compared output for output.
 ``--impl reference`` times the CPU oracle port (the reference ships no runnable CPU code for the
 student - weights only - and /root/reference is not on the GPU box) on a bounded sample.
 """
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -55,6 +58,26 @@ PWN_FLOPS_PER_SAMPLE = 25.63e6
 PWN_BYTES_PER_SAMPLE = 103609.0
 
 
+DUMP_BYTES = 60 << 20            # array data of --dump-outputs: under 64 MB with the .npy headers
+DUMP_WORKLOADS = ("pwn", "hifigan", "ragged", "e2e")
+
+
+def dump_outputs(d, arrays):
+    """Write each tensor of `arrays` as d/<name>.npy in float32.  When they exceed 60 MB together, each is replaced by a
+    fixed seeded sample of its flattened elements, and the sample's flat indices go to d/<name>_index.npy (float64)."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    arrays = {k: v.detach().to("cpu", torch.float32).contiguous() for k, v in arrays.items()}
+    total = sum(4 * v.numel() for v in arrays.values())
+    for name, v in arrays.items():
+        if total > DUMP_BYTES:          # 4 bytes of value + 8 bytes of index per kept element
+            keep = int(v.numel() * DUMP_BYTES // (3 * total))
+            idx = torch.randperm(v.numel(), generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            np.save(os.path.join(d, name + "_index.npy"), idx.to(torch.float64).numpy())
+            v = v.reshape(-1)[idx]
+        np.save(os.path.join(d, name + ".npy"), v.numpy())
+
+
 def peaks():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -75,6 +98,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", f"--id={self.index}", f"--query-gpu={q}", "--format=csv,noheader,nounits", "-lms", "100"],
                                          stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)         # a run that fails before stop() must not leave the sampler running
             self.t = threading.Thread(target=self._read, daemon=True)
             self.t.start()
         except Exception:
@@ -357,7 +381,7 @@ def run_teacher_cpu(args, desc, rank):
     rf = (C.FRONT_K - 1) + sum((C.KERNEL - 1) * C.dilation_of(i) for i in range(nb)) + 1
     mel = synthetic_mel01(1, F, seed=1234)
     c_up = C.upsample_mel(tsd, mel)
-    n = max(2, args.steps)
+    n = args.steps
     start = rf + 64                                       # steady state: the window is the full receptive field
     g = torch.Generator().manual_seed(7)
     eps = torch.randn(1, start + n + 1, generator=g)
@@ -399,7 +423,7 @@ def run_api1(args, desc, rank, local):
     dev = torch.device("cuda", local)
     torch.cuda.set_device(dev)
     out = {}
-    iters = max(5, args.steps)
+    iters = args.steps
     for arch in ("hifigan", "student"):
         weights, wdesc = load_weights(arch)
         if arch == "student":
@@ -558,6 +582,8 @@ def run_e2e(args, desc, rank, world, local):
     clocks = sampler.stop() if rank == 0 else None
     if rank == 0:
         value = total * args.steps / dt
+        if args.dump_outputs:        # rank 0's int16 audio of every string, concatenated in shard order
+            dump_outputs(args.dump_outputs, {"audio_int16": torch.cat(host)})
         print(json.dumps({
             "metric": "audio samples/sec", "value": value, "unit": "samples/s", "n_gpus": world, "steps": args.steps, "warmup": max(args.warmup, 3),
             "ms_per_step": 1e3 * dt / args.steps, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
@@ -634,6 +660,8 @@ def run_ragged(args, desc, rank, world, local):
     clocks = sampler.stop() if rank == 0 else None
     if rank == 0:
         assert all(o.numel() == voc.out_len(f) for o, f in zip(out, frames))
+        if args.dump_outputs:        # the waveform of every utterance, concatenated in input order
+            dump_outputs(args.dump_outputs, {"wav": torch.cat([o.reshape(-1) for o in out])})
         value = total * args.steps / (ms / 1e3)
         plan = cube.lpt_shard(frames, world)
         loads = [sum(frames[i] for i in p_) for p_ in plan]
@@ -670,7 +698,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--emulate-world", type=int, default=0,
                     help="ragged workload on ONE GPU: vocode only rank 0's LPT shard of a world of this size (what one rank of an N-GPU run computes)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned in its last timed step as DIR/<name>.npy (float32, at most 64 MB; "
+                         "a fixed seeded sample of larger outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "cube" or args.workload not in DUMP_WORKLOADS):
+        ap.error(f"--dump-outputs needs --impl cube and one of the workloads {', '.join(DUMP_WORKLOADS)}")
     arch, B, F, desc = WORKLOADS[args.workload]
     B = args.batch or B
     F = args.frames or F
@@ -744,8 +779,6 @@ def main():
         for k in range(args.steps):
             y = step(k)
             launches += handle.launches()
-            if k == args.steps - 1:
-                pass
         ev1.record()
         barrier()
         ms = ev0.elapsed_time(ev1)
@@ -770,6 +803,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms, e2e_ms = float(t[0]), float(t[1])
     assert bool(torch.isfinite(y).all()), "non-finite audio"
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"wav": y})
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()

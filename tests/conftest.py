@@ -68,6 +68,22 @@ def neb():
     return sd, dict(H.CONFIG_NEB)
 
 
+def neb_weights():
+    """(state_dict, config, trained?) with the shipped generator's architecture: its checkpoint when staged, else seeded
+    random weights scaled so that the tests' synthetic mel gives loud (peak 0.6 - 1.0) but unsaturated audio."""
+    from oracle import hifigan_ref as H
+    cfg = dict(H.CONFIG_NEB)
+    sd = load_staged("g_00600000")
+    if sd is not None:
+        return sd, cfg, True
+    return H.random_state_dict(cfg, seed=21, std=0.3, g_scale=0.125), cfg, False
+
+
+@pytest.fixture(scope="session")
+def neb_arch():
+    return neb_weights()
+
+
 @pytest.fixture(scope="session")
 def clarinet_weights():
     """(student_sd, teacher_sd, trained?) - shipped checkpoints when staged, else seeded random."""

@@ -31,12 +31,12 @@ def _gen(cfg, sd, dev, math=0):
 
 
 def _cached_oracle(tag, fn):
-    """CPU oracle results of the long cases are cached on disk (/tmp): the kernel-variant tests re-run this file in
-    child processes (one per env switch) and would otherwise repeat a 45 s CPU run each time."""
+    """CPU oracle results of the long cases are cached in the temporary directory, one cache per user: the kernel-variant
+    tests re-run this file in child processes (one per env switch) and would otherwise repeat a 45 s CPU run each time."""
     import hashlib
     import os
-    d = "/tmp/cube_oracle_cache"
-    os.makedirs(d, exist_ok=True)
+    import tempfile
+    d = os.path.join(tempfile.gettempdir(), f"cube_oracle_cache_{os.getuid()}")
     p = os.path.join(d, hashlib.sha1(tag.encode()).hexdigest()[:16] + ".pt")
     if os.path.exists(p):
         try:
@@ -44,8 +44,12 @@ def _cached_oracle(tag, fn):
         except Exception:
             pass
     y = fn()
-    torch.save(y, p + ".tmp")
-    os.replace(p + ".tmp", p)
+    try:
+        os.makedirs(d, exist_ok=True)
+        torch.save(y, p + f".{os.getpid()}.tmp")
+        os.replace(p + f".{os.getpid()}.tmp", p)
+    except OSError:     # a cache that cannot be written only costs time
+        pass
     return y
 
 
@@ -96,8 +100,8 @@ def test_hifigan_golden_trained(dev, neb, math):
 
 @pytest.mark.parametrize("math", MATHS)
 @pytest.mark.parametrize("level", [-5.0, 0.0, 1.0])
-def test_hifigan_trained_loudness_sweep(dev, neb, level, math):
-    sd, cfg = neb
+def test_hifigan_trained_loudness_sweep(dev, neb_arch, level, math):
+    sd, cfg, _ = neb_arch
     mel = H.synthetic_mel(2, 40, seed=1237 + int(level), level=level)
     ref = H.generator_forward(sd, cfg, mel)
     g = _gen(cfg, sd, dev, math)
@@ -199,10 +203,10 @@ def test_forward_host_graph_replay(dev):
 
 
 @pytest.mark.parametrize("math", MATHS)
-def test_hifigan_full_size_properties(dev, neb, math):
+def test_hifigan_full_size_properties(dev, neb_arch, math):
     """BASELINE config 3 shape (10 s utterances) through size-independent properties: batch items are
     independent and a long utterance equals the same utterance inside a padded batch."""
-    sd, cfg = neb
+    sd, cfg, _ = neb_arch
     g = _gen(cfg, sd, dev, math)
     F = 919
     mel = H.synthetic_mel(2, F, seed=77)
@@ -230,13 +234,14 @@ def test_hifigan_full_size_properties(dev, neb, math):
 
 @pytest.mark.parametrize("math", MATHS)
 @pytest.mark.parametrize("level", [0.0, 1.0])
-def test_hifigan_full_length_oracle(dev, neb, level, math):
+def test_hifigan_full_length_oracle(dev, neb_arch, level, math):
     """BASELINE configs[2] geometry, compared with the oracle over the WHOLE 10-s utterance (F = 919, T = 220 656), the
-    shipped generator, speech level (0) and the saturating corner (+1), both math modes.  hifigan/models.py:100-116."""
-    sd, cfg = neb
+    shipped generator (seeded weights of its architecture when the checkpoint is not staged), speech level (0) and the
+    saturating corner (+1), both math modes.  hifigan/models.py:100-116."""
+    sd, cfg, trained = neb_arch
     F = 919
     mel = H.synthetic_mel(2, F, seed=177 + int(level), level=level)
-    ref = _cached_oracle(f"hifigan_neb_full_F{F}_lvl{level}_seed{177 + int(level)}", lambda: H.generator_forward(sd, cfg, mel))
+    ref = _cached_oracle(f"hifigan_neb_full_F{F}_lvl{level}_seed{177 + int(level)}_trained{trained}", lambda: H.generator_forward(sd, cfg, mel))
     g = _gen(cfg, sd, dev, math)
     with torch.no_grad():
         y = g(mel.to(dev)).cpu()
@@ -710,12 +715,12 @@ def test_mel_cube_flavour(dev):
         cube.MelSpectrogram(1024, 80, 24000, 250, 1024, 0, 12000)(torch.zeros(1, 4000, device=dev))   # hop not a multiple of 4
 
 
-def test_mel_copy_synthesis_chain(dev, neb):
+def test_mel_copy_synthesis_chain(dev, neb_arch):
     """wav -> device mel -> HiFi-GAN (the hifigan/inference.py:26-45 copy-synthesis chain) stays on the GPU and matches
     the same chain through the CPU oracles."""
     import tts_cube_b200 as cube
     from oracle import mel_ref as M
-    sd, cfg = neb
+    sd, cfg, _ = neb_arch
     y = M.test_signal(1, 16 * 256, seed=12)
     args = (1024, 80, 22050, 256, 1024, 0, 8000)
     mel = cube.mel_spectrogram(y.to(dev), *args)
@@ -730,14 +735,10 @@ def test_mel_copy_synthesis_chain(dev, neb):
 _BITS_SCRIPT = """
 import hashlib, sys, torch
 sys.path[:0] = [%r, %r]
-from conftest import load_staged
+from conftest import neb_weights
 from oracle import hifigan_ref as H
 import tts_cube_b200 as cube
-sd = load_staged("g_00600000")
-cfg = dict(H.CONFIG_NEB)
-if sd is None:   # no trained checkpoint staged: seeded random weights, 64- and 32-channel stages included
-    cfg = dict(H.CONFIG_V1, upsample_initial_channel=128)
-    sd = H.random_state_dict(cfg, seed=21, std=0.3, g_scale=0.25)
+sd, cfg, _ = neb_weights()
 g = cube.CubeGenerator(cfg, math=1).to("cuda:0"); g.load_state_dict(sd); g.eval()
 mel = H.synthetic_mel(3, 70, seed=5)
 with torch.no_grad():

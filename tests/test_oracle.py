@@ -186,10 +186,12 @@ def test_teacher_generate_is_consistent_with_teacher_forcing():
 
 
 def test_upsamplenet_oracle_matches_reference():
-    """cube/networks/modules.py:317-343: the restatement equals the reference-run golden bit for bit"""
+    """cube/networks/modules.py:317-343: the restatement equals the reference-run golden bit for bit on the CPU code path
+    the golden was made with.  ATen's conv and tanh round differently under another oneDNN ISA or vector width (both
+    follow the host CPU), which moves outputs by up to two ulps of their peak; the tolerance is twice that."""
     from oracle import wavernn_ref as R
     d = load_golden("upsamplenet.npz")
     sd = golden_weights(d)
     y = R.upsamplenet_forward(sd, torch.from_numpy(d["c"]), [int(s) for s in d["scales"]], int(d["kernel_size"]))
     assert y.shape == d["y"].shape == (2, 24, 9 * 16)
-    assert float((y - torch.from_numpy(d["y"])).abs().max()) == 0.0
+    assert float((y - torch.from_numpy(d["y"])).abs().max()) <= 4 * float(np.spacing(np.abs(d["y"]).max()))
