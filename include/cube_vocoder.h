@@ -117,6 +117,20 @@ int64_t cube_voc_out_len(const cube_voc_t* h, int64_t n_frames);
 int cube_voc_forward(cube_voc_t* h, const float* mel, const int32_t* n_frames, const float* noise,
                      float* wav, int16_t* wav_i16, int B, int64_t Fmax, cube_stream_t stream);
 
+/* Streaming geometry of a HiFi-GAN config (no handle, no device): the mel frames [*f0, *f1) that output samples [s0, s1)
+ * depend on, by exact interval propagation through conv_pre, every ConvTranspose1d (input i reaches outputs i*u - pad + j,
+ * j < K) and ResBlock step, and conv_post.  *f0 is clipped at 0 (earlier rows are zero padding); *f1 is not clipped above,
+ * so a caller holding N frames may emit [s0, s1) once *f1 <= N.  Fails for other archs and for s0 < 0 or s0 >= s1. */
+int cube_voc_hifigan_support(const cube_voc_config* cfg, int64_t s0, int64_t s1, int64_t* f0, int64_t* f1);
+
+/* cube_voc_forward for HiFi-GAN handles that writes only samples [out_begin[b], out_end[b]) of item b (HOST arrays [B]);
+ * every other element of wav / wav_i16 is left untouched.  Same arguments and layout as cube_voc_forward.  The requested
+ * samples are bit-identical to what cube_voc_forward computes for the same mel: every launch schedules only the rows its
+ * consumers read (tensor-core path), and no row's arithmetic depends on the tile it falls in.  Fails for other archs and
+ * for a range that is empty or outside [0, cube_voc_out_len(n_frames[b])). */
+int cube_voc_forward_range(cube_voc_t* h, const float* mel, const int32_t* n_frames, const int64_t* out_begin,
+                           const int64_t* out_end, float* wav, int16_t* wav_i16, int B, int64_t Fmax, cube_stream_t stream);
+
 /* Same call with HOST buffers (pinned or pageable): H2D of mel/noise, forward, D2H of the audio;
  * synchronous.  This is the end-to-end form of `cube(text)`'s vocoder leg
  * (cube/api.py:60-65: .to(device) ... .detach().cpu().numpy(), *32767 -> int16).

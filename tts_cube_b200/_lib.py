@@ -68,6 +68,10 @@ SYMBOLS = {
     "cube_voc_out_len": (C.c_int64, [_P, C.c_int64]),
     "cube_voc_forward": (C.c_int, [_P, _P, _P, _P, _P, _P, C.c_int, C.c_int64, _P]),
     "cube_voc_forward_host": (C.c_int, [_P, _P, _P, _P, _P, _P, C.c_int, C.c_int64]),
+    "cube_voc_hifigan_support": (C.c_int, [C.POINTER(VocConfig), C.c_int64, C.c_int64, C.POINTER(C.c_int64),
+                                           C.POINTER(C.c_int64)]),
+    "cube_voc_forward_range": (C.c_int, [_P, _P, _P, C.POINTER(C.c_int64), C.POINTER(C.c_int64), _P, _P, C.c_int,
+                                         C.c_int64, _P]),
     "cube_voc_get_cond": (C.c_int, [_P, _P, C.c_int, C.c_int64, _P]),
     "cube_wavernn_out_len": (C.c_int64, [_P, C.c_int64, C.c_int64]),
     "cube_wavernn_forward": (C.c_int, [_P, _P, _P, _P, _P, C.c_int, C.c_int64, C.c_int64, _P]),

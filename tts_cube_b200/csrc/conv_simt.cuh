@@ -245,6 +245,8 @@ struct SmallP {
   const float* z; long long z_bstride;   // IAF: z_old
   int ci_chunk;
   int epi;
+  int row0, nrows;                       // output steps [row0, row0 + nrows) are computed (nrows = 0: all L_out)
+  const int* out_rng;                    // [B][2] device: store only steps [rng[2b], rng[2b+1]) of item b, or null
 };
 
 template <int MO, int TPT>  // TPT = time steps per thread
@@ -252,7 +254,7 @@ __global__ void __launch_bounds__(256) conv_small_kernel(const SmallP p) {
   constexpr int BN = 256 * TPT;
   extern __shared__ __align__(16) float smem[];
   const int tid = threadIdx.x;
-  const int q0 = blockIdx.x * BN;
+  const int q0 = p.row0 + blockIdx.x * BN;
   const int b = blockIdx.y;
   const int span = (p.taps - 1) * p.dil;
   const int XW = BN + span;
@@ -325,6 +327,7 @@ __global__ void __launch_bounds__(256) conv_small_kernel(const SmallP p) {
   for (int j = 0; j < TPT; ++j) {
     const int t = q0 + tid + 256 * j;
     if (t >= p.L_out) continue;
+    if (p.out_rng && (t < p.out_rng[2 * b] || t >= p.out_rng[2 * b + 1])) continue;
     if (p.epi == SEPI_IAF) {
       // (mu, logs) at t drive sample t+1:  z'[t+1] = z[t+1]*exp(logs[t]) + mu[t],  z'[0] = 0
       if (MO >= 2) {

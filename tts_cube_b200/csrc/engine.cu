@@ -146,6 +146,7 @@ struct cube_voc {
   struct UpNet { PackedConv conv[3]; std::vector<PackedConv> up; std::vector<int> J; } upnet;
   // last-forward geometry (for get_cond)
   int last_B = 0; int64_t last_T = 0;
+  std::vector<int> h_rng;                   // cube_voc_forward_range: [B][2] sample ranges (pageable, as h_lens)
 };
 
 namespace cube {
@@ -540,7 +541,7 @@ struct Launcher {
     if (cic < 1) cic = 1;
     p.ci_chunk = cic;
     const size_t smem = ((size_t)((p.C * p.taps * MO + 3) & ~3) + (size_t)cic * XP) * sizeof(float);
-    dim3 grid((p.L_out + BN - 1) / BN, B);
+    dim3 grid(((p.nrows > 0 ? p.nrows : p.L_out) + BN - 1) / BN, B);
     static bool a1[64] = {false}, a2[64] = {false};
     const int dv = h->device & 63;
     if (MO == 1) {
@@ -793,6 +794,84 @@ static int64_t hifigan_len(const cube_voc_config& c, int64_t L, int upto) {
   return L;
 }
 
+// ------------------------------------------------------------------------------------------------
+// streaming geometry: the rows of every layer that output samples [s0, s1) depend on
+// ------------------------------------------------------------------------------------------------
+struct RowRange { int64_t a, b; };   // rows [a, b)
+
+struct HifiganPlan {
+  RowRange mel, pre, post;                                // mel frames, conv_pre output rows, conv_post samples
+  std::vector<RowRange> ups;                              // [stage]: ConvTranspose1d output rows its ResBlocks read
+  std::vector<std::vector<std::vector<RowRange>>> step;   // [stage][resblock][m]: output rows of ResBlock step m
+};
+
+static inline int64_t fdiv(int64_t a, int64_t b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
+
+// ResBlock step m of kernel k: rows of its input that one output row reaches, left and right
+static void step_halo(const cube_voc_config& c, int k, int d, int64_t* hl, int64_t* hr) {
+  const int64_t l1 = (int64_t)(k * d - d) / 2, r1 = (int64_t)(k - 1) * d - l1;   // conv1 (or ResBlock2's only conv), "same" pad
+  const int64_t l2 = (k - 1) / 2, r2 = (k - 1) - l2;                            // ResBlock1's conv2, dilation 1
+  *hl = c.resblock_type == 1 ? l1 + l2 : l1;
+  *hr = c.resblock_type == 1 ? r1 + r2 : r1;
+}
+
+// Per-phase rows q of ups[i] whose outputs t = q*u + r - pad (r < u) meet output rows [a, b)
+static RowRange ups_phase_rows(const cube_voc_config& c, int i, RowRange t) {
+  const int u = c.upsample_rates[i], pad = (c.upsample_kernel_sizes[i] - u) / 2;
+  return {fdiv(t.a + pad, u), fdiv(t.b - 1 + pad, u) + 1};
+}
+
+// Walks the generator backward from output samples [s0, s1).  Every level's range is clipped below at 0 (rows before the
+// start are the convs' zero padding and depend on nothing) and, if lens is given, above at lens[l] (l = 0: frames,
+// l = n_ups: samples).  phase_reads: the ConvTranspose1d input is what the per-phase kernels read (J = ceil(K/u) taps per
+// phase; where K % u != 0 the taps past K hold zero weights but their rows are still multiplied), else the rows with a
+// non-zero weight: input i reaches outputs i*u - pad + j, j < K.
+static void hifigan_plan(const cube_voc_config& c, int64_t s0, int64_t s1, const int64_t* lens, bool phase_reads,
+                         HifiganPlan* P) {
+  const int nU = c.n_ups, nk = c.n_resblock_kernels;
+  auto clip = [&](RowRange r, int l) {
+    r.a = std::max<int64_t>(r.a, 0);
+    if (lens) r.b = std::min<int64_t>(r.b, lens[l]);
+    if (r.b < r.a) r.b = r.a;
+    return r;
+  };
+  P->ups.assign(nU, {0, 0});
+  P->step.assign(nU, std::vector<std::vector<RowRange>>(nk));
+  RowRange x = clip({s0, s1}, nU);
+  P->post = x;
+  x = clip({x.a - 3, x.b + 3}, nU);                        // conv_post: k = 7, pad 3
+  for (int i = nU - 1; i >= 0; --i) {                      // x = rows of stage i's output (the ResBlock average)
+    RowRange un{INT64_MAX, INT64_MIN};
+    for (int j = 0; j < nk; ++j) {
+      const int k = c.resblock_kernel_sizes[j], nd = c.n_dilations[j];
+      P->step[i][j].assign(nd, {0, 0});
+      RowRange r = x;                                      // every ResBlock's last step covers the stage output range
+      for (int m = nd - 1; m >= 0; --m) {
+        P->step[i][j][m] = r;
+        int64_t hl, hr;
+        step_halo(c, k, c.resblock_dilations[j][m], &hl, &hr);
+        r = clip({r.a - hl, r.b + hr}, i + 1);
+      }
+      un.a = std::min(un.a, r.a); un.b = std::max(un.b, r.b);
+    }
+    P->ups[i] = un;                                        // the three ResBlocks share the ups output: the widest need
+    const int u = c.upsample_rates[i], K = c.upsample_kernel_sizes[i], pad = (K - u) / 2;
+    if (phase_reads) {
+      const RowRange q = ups_phase_rows(c, i, un);
+      const int J = (K + u - 1) / u;
+      x = clip({q.a - (J - 1), q.b}, i);
+    } else {
+      x = clip({fdiv(un.a + pad - K + 1 + u - 1, u), fdiv(un.b - 1 + pad, u) + 1}, i);
+    }
+  }
+  P->pre = x;
+  P->mel = clip({x.a - 3, x.b + 3}, 0);                   // conv_pre: k = 7, pad 3
+}
+
+// what cube_voc_forward_range asks of the HiFi-GAN forward: samples [s0, s1) of the batch (the union of the items'
+// ranges) and the per-item ranges the conv_post stores are masked to
+struct RangeReq { int64_t s0, s1; const int* d_rng; };
+
 // valid length of every utterance at every level of the network -> h->h_lens [nlevels][B] (host only)
 static int fill_lens(cube_voc* h, const int32_t* n_frames, int B, int64_t Fmax, int nlevels) {
   const size_t need = (size_t)nlevels * B;
@@ -848,12 +927,13 @@ static int upload_lens(cube_voc* h, const int32_t* n_frames, int B, int64_t Fmax
 }
 
 static int forward_hifigan_tc(cube_voc* h, const float* mel, const int32_t* n_frames, float* wav, int16_t* wav16,
-                              int B, int64_t Fmax, cudaStream_t st);
+                              int B, int64_t Fmax, cudaStream_t st, const RangeReq* rq);
 
+// rq: cube_voc_forward_range.  The fp32 path computes the whole window and only crops and masks conv_post
 static int forward_hifigan(cube_voc* h, const float* mel, const int32_t* n_frames, float* wav, int16_t* wav16,
-                           int B, int64_t Fmax, cudaStream_t st) {
+                           int B, int64_t Fmax, cudaStream_t st, const RangeReq* rq = nullptr) {
   const cube_voc_config& c = h->cfg;
-  if (c.math == CUBE_MATH_TC_SPLIT16) return forward_hifigan_tc(h, mel, n_frames, wav, wav16, B, Fmax, st);
+  if (c.math == CUBE_MATH_TC_SPLIT16) return forward_hifigan_tc(h, mel, n_frames, wav, wav16, B, Fmax, st, rq);
   const int nU = c.n_ups, nk = c.n_resblock_kernels;
   std::vector<int64_t> L(nU + 1);
   for (int i = 0; i <= nU; ++i) L[i] = hifigan_len(c, Fmax, i);
@@ -963,6 +1043,7 @@ static int forward_hifigan(cube_voc* h, const float* mel, const int32_t* n_frame
     p.W = h->conv_post_w.W; p.bias = h->conv_post_w.bias;
     p.out_lens = h->d_lens + (size_t)nU * B; p.L_out = Lo;
     p.out = wav; p.out_bstride = Lo; p.out_i16 = wav16; p.epi = SEPI_TANH;
+    if (rq) { p.row0 = (int)rq->s0; p.nrows = (int)(rq->s1 - rq->s0); p.out_rng = rq->d_rng; }
     lx.small(p, B, 1);
     lx.end();
   }
@@ -1061,7 +1142,7 @@ static int launch_rbstep_v(cube_voc* h, tc::RbParams& rp, cudaStream_t st) {
     attr[h->device & 63] = true;
   }
   const int r_out = NSUB * tc::BM - (rp.k - 1);
-  rp.t_tiles = (rp.L + r_out - 1) / r_out;
+  rp.t_tiles = ((rp.nrows > 0 ? rp.nrows : rp.L) + r_out - 1) / r_out;
   const long long tiles = (long long)rp.t_tiles * rp.B;
   const int grid = (int)std::min<long long>(tiles, h->sm_count);
   tc::tc_rbstep_kernel<C, NSUB, PK><<<grid, tc::RB_THREADS, Cfg::SMEM, st>>>(rp);
@@ -1085,10 +1166,12 @@ static int wide_mode() {
 }
 static bool use_wide() { return wide_mode() > 0; }
 
-// tp.T = rows per batch item; fills t_tiles for the chosen variant and launches
+// tp.T = rows per batch item, of which tp.nrows from tp.row0 are scheduled (0: all); fills t_tiles for the chosen variant
+// and launches
 template <int TN, int MS = 0>
 static void launch_tc_t(cube_voc* h, tc::TcParams& tp, cudaStream_t st) {
   const int nph = tp.nphase > 0 ? tp.nphase : 1;
+  const int rows = tp.nrows > 0 ? tp.nrows : tp.T;
   if (MS == 0 && use_cg2()) {
     static bool attr2[64] = {false};
     if (!attr2[h->device & 63]) {
@@ -1096,7 +1179,7 @@ static void launch_tc_t(cube_voc* h, tc::TcParams& tp, cudaStream_t st) {
       attr2[h->device & 63] = true;
     }
     constexpr int rows2 = 2 * tc::BM * tc::Cfg<TN, true>::MSUB;
-    tp.t_tiles = (tp.T + rows2 - 1) / rows2;
+    tp.t_tiles = (rows + rows2 - 1) / rows2;
     const long long tiles = (long long)tp.n_tiles * tp.t_tiles * tp.B * nph;
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
@@ -1112,7 +1195,7 @@ static void launch_tc_t(cube_voc* h, tc::TcParams& tp, cudaStream_t st) {
     return;
   }
   constexpr int rows1 = tc::BM * tc::Cfg<TN, false, MS>::MSUB;
-  tp.t_tiles = (tp.T + rows1 - 1) / rows1;
+  tp.t_tiles = (rows + rows1 - 1) / rows1;
   const long long tiles = (long long)tp.n_tiles * tp.t_tiles * tp.B * nph;
   const int grid = (int)std::min<long long>(tiles, h->sm_count);
   if (use_win(h)) {
@@ -1160,7 +1243,9 @@ static void launch_tc_t(cube_voc* h, tc::TcParams& tp, cudaStream_t st) {
 }
 
 // Two sub-tiles per scheduled tile halve the number of tiles: worth it only while 128-row tiles would fill the SMs more than
-// twice over.  At batch 1 the 128-channel stage of a 10-s utterance has 108 such tiles for 148 SMs - as 54 double tiles every
+// twice over.  Decided from the whole tensor (tp.T), never from a cropped row range: the two-sub-tile variant accumulates
+// a_hi*w_hi, a_hi*w_lo and a_lo*w_hi in one accumulator while the 128-column tile sums a_hi*w_lo separately (CAT in
+// tc_conv.cuh), so the variants differ in the last bits and cube_voc_forward_range must pick what cube_voc_forward picks.  At batch 1 the 128-channel stage of a 10-s utterance has 108 such tiles for 148 SMs - as 54 double tiles every
 // conv of the stage would take twice as long (the latency the `api1` workload measures).
 static bool wide_pays(const cube_voc* h, const tc::TcParams& tp) {
   const long long nph = tp.nphase > 0 ? tp.nphase : 1;
@@ -1176,13 +1261,21 @@ static void launch_tc_bn(cube_voc* h, int bn, tc::TcParams& tp, cudaStream_t st)
   else launch_tc_t<32>(h, tp, st);
 }
 
+// rq (cube_voc_forward_range): every launch schedules only the rows its consumers read (hifigan_plan over the buffer
+// lengths, never an item's valid length: rows between the two are written as zero and read as the next conv's padding)
 static int forward_hifigan_tc(cube_voc* h, const float* mel, const int32_t* n_frames, float* wav, int16_t* wav16,
-                              int B, int64_t Fmax, cudaStream_t st) {
+                              int B, int64_t Fmax, cudaStream_t st, const RangeReq* rq) {
   const cube_voc_config& c = h->cfg;
   const int nU = c.n_ups, nk = c.n_resblock_kernels;
   std::vector<int64_t> L(nU + 1);
   for (int i = 0; i <= nU; ++i) L[i] = hifigan_len(c, Fmax, i);
   if (L[nU] > 0x7fffffffLL / 2) return fail("utterance too long");
+  HifiganPlan plan;
+  if (rq) hifigan_plan(c, rq->s0, rq->s1, L.data(), true, &plan);
+  auto crop = [&](auto& prm, RowRange r) {    // TcParams / RbParams: schedule rows [r.a, r.b) only
+    if (!rq) return;
+    prm.row0 = (int)r.a; prm.nrows = (int)std::max<int64_t>(r.b - r.a, 1);
+  };
   if (upload_lens(h, n_frames, B, Fmax, nU + 1, st)) return 1;
   const int C0 = c.upsample_initial_channel;
   size_t stage_max = (size_t)C0 * L[0];
@@ -1216,7 +1309,9 @@ static int forward_hifigan_tc(cube_voc* h, const float* mel, const int32_t* n_fr
   };
   {  // mel -> fp16 planes (pad frames masked), then conv_pre; its output is stored lrelu'd for ups[0]
     lx.begin("to_hl16");
-    tc::to_hl16_kernel<<<dim3(((int)Fmax + 31) / 32, (c.num_mels + 31) / 32, B), 256, 0, st>>>(mel, M16, B, c.num_mels, (int)Fmax, h->d_lens, PS);
+    const RowRange mr = rq ? plan.mel : RowRange{0, Fmax};
+    tc::to_hl16_kernel<<<dim3((int)(mr.b - mr.a + 31) / 32, (c.num_mels + 31) / 32, B), 256, 0, st>>>(mel, M16, B, c.num_mels, (int)Fmax,
+                                                                                                     h->d_lens, PS, (int)mr.a);
     lx.check();
     lx.end();
     lx.begin("conv_pre");
@@ -1224,6 +1319,7 @@ static int forward_hifigan_tc(cube_voc* h, const float* mel, const int32_t* n_fr
     if (base_params(h->tc_conv_pre, M16, (int)L[0], c.num_mels, (int)L[0], (int)L[0], C0, h->d_lens, tp)) return 1;
     tp.seg[0].dil = 1; tp.seg[0].off0 = -3;
     tp.out16 = P0;
+    crop(tp, plan.pre);
     launch_tc_bn(h, h->tc_conv_pre.bn, tp, st);
     lx.check();
     lx.end();
@@ -1241,6 +1337,10 @@ static int forward_hifigan_tc(cube_voc* h, const float* mel, const int32_t* n_fr
       tp.ostride = u;
       for (int r = 0; r < u; ++r) tp.ooff[r] = r - pad;
       tp.out16 = U;
+      if (rq) {   // per-phase rows q (output t = q*u + r - pad) of the ResBlocks' widest need
+        const RowRange q = ups_phase_rows(c, i, plan.ups[i]);
+        crop(tp, RowRange{std::max<int64_t>(q.a, 0), std::min<int64_t>(q.b, tp.T)});
+      }
       launch_tc_bn(h, h->tc_ups[i].bn, tp, st);
       lx.check();
       lx.end();
@@ -1267,6 +1367,7 @@ static int forward_hifigan_tc(cube_voc* h, const float* mel, const int32_t* n_fr
         rp.W2 = w2.Wimg; rp.inv2 = w2.inv_scale; rp.bias2 = w2.bias;
         rp.k = k; rp.dil = d; rp.B = B; rp.L = Lo; rp.lens = lens_out;
         rp.x16 = xcur; rp.slope = LR; rp.inv_slope = 1.f / LR;
+        if (rq) crop(rp, plan.step[i][j][m]);
         const bool last = (m == nd - 1);
         __half* outp = (m & 1) ? T1 : R;
         if (!last) {
@@ -1292,6 +1393,10 @@ static int forward_hifigan_tc(cube_voc* h, const float* mel, const int32_t* n_fr
           if (base_params(h->tc_c1[idx][m], xcur, Lo, ch, Lo, Lo, ch, lens_out, tp)) return 1;
           tp.seg[0].dil = d; tp.seg[0].off0 = -((k * d - d) / 2);
           tp.out16 = T1;
+          if (rq) {   // conv2's input: the step's rows and conv2's halo
+            const RowRange s = plan.step[i][j][m];
+            crop(tp, RowRange{std::max<int64_t>(s.a - (k - 1) / 2, 0), std::min<int64_t>(s.b + (k - 1) - (k - 1) / 2, Lo)});
+          }
           launch_tc_bn(h, h->tc_c1[idx][m].bn, tp, st);
           lx.check();
           lx.end();
@@ -1302,6 +1407,7 @@ static int forward_hifigan_tc(cube_voc* h, const float* mel, const int32_t* n_fr
           if (base_params(h->tc_c2[idx][m], T1, Lo, ch, Lo, Lo, ch, lens_out, tp)) return 1;
           tp.seg[0].dil = 1; tp.seg[0].off0 = -((k - 1) / 2);
           tp.res16 = xcur;
+          if (rq) crop(tp, plan.step[i][j][m]);
           const bool last = (m == nd - 1);
           if (!last) {
             tp.out16 = R;
@@ -1331,6 +1437,7 @@ static int forward_hifigan_tc(cube_voc* h, const float* mel, const int32_t* n_fr
     p.W = h->conv_post_w.W; p.bias = h->conv_post_w.bias;
     p.out_lens = h->d_lens + (size_t)nU * B; p.L_out = Lo;
     p.out = wav; p.out_bstride = Lo; p.out_i16 = wav16; p.epi = SEPI_TANH;
+    if (rq) { p.row0 = (int)plan.post.a; p.nrows = (int)(plan.post.b - plan.post.a); p.out_rng = rq->d_rng; }
     lx.small(p, B, 1);
     lx.end();
   }
@@ -2044,6 +2151,58 @@ int cube_voc_forward(cube_voc_t* h, const float* mel, const int32_t* n_frames, c
     return forward_upsamplenet(h, mel, n_frames, wav, B, Fmax, st);
   }
   return forward_student(h, mel, n_frames, noise, wav, wav_i16, B, Fmax, st);
+}
+
+int cube_voc_hifigan_support(const cube_voc_config* cfg, int64_t s0, int64_t s1, int64_t* f0, int64_t* f1) {
+  if (!cfg || !f0 || !f1) return fail("null argument");
+  if (cfg->struct_size != sizeof(cube_voc_config))
+    return fail("cube_voc_config.struct_size = %u but this library's struct is %zu bytes", cfg->struct_size, sizeof(cube_voc_config));
+  if (cfg->arch != CUBE_VOC_HIFIGAN) return fail("sample support is defined for HiFi-GAN configs only");
+  if (cfg->n_ups < 1 || cfg->n_ups > CUBE_MAX_UPS || cfg->n_resblock_kernels < 1 || cfg->n_resblock_kernels > CUBE_MAX_RBK)
+    return fail("bad HiFi-GAN config (n_ups=%d, n_resblock_kernels=%d)", cfg->n_ups, cfg->n_resblock_kernels);
+  for (int i = 0; i < cfg->n_ups; ++i)
+    if (cfg->upsample_rates[i] < 1 || cfg->upsample_kernel_sizes[i] < cfg->upsample_rates[i])
+      return fail("bad upsample stage %d (rate %d, kernel %d)", i, cfg->upsample_rates[i], cfg->upsample_kernel_sizes[i]);
+  for (int j = 0; j < cfg->n_resblock_kernels; ++j)
+    if (cfg->resblock_kernel_sizes[j] < 1 || cfg->n_dilations[j] < 1 || cfg->n_dilations[j] > CUBE_MAX_DIL)
+      return fail("bad ResBlock %d", j);
+  if (s0 < 0 || s0 >= s1) return fail("empty or negative sample range [%lld, %lld)", (long long)s0, (long long)s1);
+  HifiganPlan P;
+  hifigan_plan(*cfg, s0, s1, nullptr, false, &P);
+  *f0 = P.mel.a; *f1 = P.mel.b;
+  return 0;
+}
+
+int cube_voc_forward_range(cube_voc_t* h, const float* mel, const int32_t* n_frames, const int64_t* out_begin,
+                           const int64_t* out_end, float* wav, int16_t* wav_i16, int B, int64_t Fmax, cube_stream_t stream) {
+  if (!h) return fail("null handle");
+  if (h->cfg.arch != CUBE_VOC_HIFIGAN) return fail("the sample-range forward is defined for HiFi-GAN handles only");
+  if (!h->finalized) return fail("forward before finalize");
+  if (!mel || !wav || !out_begin || !out_end) return fail("null mel/wav/out_begin/out_end");
+  if (B < 1 || Fmax < 1) return fail("empty batch (B=%d, Fmax=%lld)", B, (long long)Fmax);
+  int64_t s0 = INT64_MAX, s1 = 0;
+  h->h_rng.resize((size_t)2 * B);
+  for (int b = 0; b < B; ++b) {
+    const int64_t f = n_frames ? n_frames[b] : Fmax;
+    if (f < 0 || f > Fmax) return fail("n_frames[%d]=%lld outside [0, %lld]", b, (long long)f, (long long)Fmax);
+    const int64_t T = f == 0 ? 0 : hifigan_len(h->cfg, f, h->cfg.n_ups);
+    if (out_begin[b] < 0 || out_begin[b] >= out_end[b] || out_end[b] > T)
+      return fail("sample range [%lld, %lld) of item %d is empty or outside [0, %lld)", (long long)out_begin[b],
+                  (long long)out_end[b], b, (long long)T);
+    s0 = std::min(s0, out_begin[b]); s1 = std::max(s1, out_end[b]);
+    h->h_rng[2 * b] = (int)out_begin[b]; h->h_rng[2 * b + 1] = (int)out_end[b];
+  }
+  if (hifigan_len(h->cfg, Fmax, h->cfg.n_ups) > 0x7fffffffLL / 2) return fail("utterance too long");
+  if (ensure_device(h)) return 1;
+  h->launches = 0;
+  for (auto& r : h->prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
+  h->prof.clear();
+  cudaStream_t st = (cudaStream_t)stream;
+  float* d_rng;
+  if (ws_get(h, "rng", (size_t)2 * B, &d_rng)) return 1;   // int32 in a float-sized buffer
+  CU_TRY(cudaMemcpyAsync(d_rng, h->h_rng.data(), (size_t)2 * B * sizeof(int), cudaMemcpyHostToDevice, st));
+  const RangeReq rq{s0, s1, (const int*)d_rng};
+  return forward_hifigan(h, mel, n_frames, wav, wav_i16, B, Fmax, st, &rq);
 }
 
 // CUBE_GRAPH=0 disables the CUDA-graph replay of the host-buffer call

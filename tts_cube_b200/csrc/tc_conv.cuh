@@ -143,6 +143,7 @@ struct TcParams {
   float* acc32; int acc_mode; float acc_div; int acc_store;
   __half* out16b;
   int lean;                 // window mode: 1 = the MMA thread's short instruction stream ("lean issue" in the kernel)
+  int row0, nrows;          // scheduled rows [row0, row0 + nrows) of q (nrows = 0: all T); the same for every batch item
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -513,7 +514,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_conv_kernel(const __grid_co
         int rest = tile / p.n_tiles;
         const int ph = rest % nphase; rest /= nphase;
         const int tt = rest % p.t_tiles, b = rest / p.t_tiles;
-        const int t0 = tt * TILE_ROWS;
+        const int t0 = p.row0 + tt * TILE_ROWS;
         const __half* wt = p.Wimg + (size_t)ph * p.w_phase_stride + (size_t)nt * p.nchunks_total * 2 * (BN * BK);
         for (int s = 0; s < p.nseg; ++s) {
           const TcSeg sg = p.seg[s];
@@ -549,7 +550,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_conv_kernel(const __grid_co
         int rest = tile / p.n_tiles;
         const int ph = rest % nphase; rest /= nphase;
         const int tt = rest % p.t_tiles, b = rest / p.t_tiles;
-        const int t0 = tt * TILE_ROWS + (int)crank * CTA_ROWS;
+        const int t0 = p.row0 + tt * TILE_ROWS + (int)crank * CTA_ROWS;
         const __half* wt = p.Wimg + (size_t)ph * p.w_phase_stride + (size_t)nt * p.nchunks_total * 2 * (BN * BK);
         int chunk = 0;
         for (int s = 0; s < p.nseg; ++s) {
@@ -775,7 +776,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_conv_kernel(const __grid_co
       int rest = tile / p.n_tiles;
       const int ph = rest % nphase; rest /= nphase;
       const int tt = rest % p.t_tiles, b = rest / p.t_tiles;
-      const int t = tt * TILE_ROWS + (int)crank * CTA_ROWS + msub * BM + row;
+      const int t = p.row0 + tt * TILE_ROWS + (int)crank * CTA_ROWS + msub * BM + row;
       const uint32_t acc = titer & 1, aph = (titer >> 1) & 1;
       // per-column (de-scale, bias) of this tile -> smem.  For the gate the exp2 pre-factors are
       // folded in: filter columns carry 2*log2(e) (-> 2^a = e^{2f}), gate columns -log2(e) (-> e^{-g}).
@@ -1082,9 +1083,10 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_conv_kernel(const __grid_co
 // through shared memory so both sides are coalesced.
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) to_hl16_kernel(const float* __restrict__ src, __half* __restrict__ dst, int B, int C, int T,
-                                                      const int* __restrict__ lens = nullptr, float scale = 1.f) {
+                                                      const int* __restrict__ lens = nullptr, float scale = 1.f,
+                                                      int row0 = 0) {
   __shared__ float tile[32][33];
-  const int b = blockIdx.z, c0 = blockIdx.y * 32, t0 = blockIdx.x * 32;
+  const int b = blockIdx.z, c0 = blockIdx.y * 32, t0 = row0 + blockIdx.x * 32;   // grid.x covers the rows wanted from row0
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;  // 32 x 8
   for (int i = ty; i < 32; i += 8) {
     const int c = c0 + i, t = t0 + tx;

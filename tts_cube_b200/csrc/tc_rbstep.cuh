@@ -63,7 +63,8 @@ struct RbParams {
   const float* inv1; const float* bias1;   // [C] power-of-two de-scale and bias of conv1
   const float* inv2; const float* bias2;
   int k, dil;                 // conv1: k taps at dilation dil; conv2: k taps at dilation 1; "same" padding
-  int B, L, t_tiles;          // L rows per batch item; t_tiles = ceil(L / (NSUB*128 - (k-1)))
+  int B, L, t_tiles;          // L rows per batch item; t_tiles = ceil(nrows / (NSUB*128 - (k-1)))
+  int row0, nrows;            // output rows [row0, row0 + nrows) are scheduled (nrows = 0: all L); the same for every item
   const int* lens;            // [B] valid rows (rows >= len are written as zero) or null
   const __half* x16;          // the same input planes, for the residual (x = inverse leaky-ReLU of the stored value)
   float slope, inv_slope;     // 0.1, 10
@@ -171,7 +172,7 @@ __global__ void __launch_bounds__(RB_THREADS, 1) tc_rbstep_kernel(const __grid_c
         else if (!mbar_test_wait(xempty, par)) return;      // a probe, never a sleep: this thread is also feeding the weight ring
         const int tile = (int)blockIdx.x + x_next * (int)gridDim.x;
         const int tt = tile % p.t_tiles, b = tile / p.t_tiles;
-        const int r0 = tt * R_OUT - h2 - h1;                 // first row of the x window
+        const int r0 = p.row0 + tt * R_OUT - h2 - h1;                 // first row of the x window
         mbar_expect_tx(xfull, Cfg::XWIN);
         for (int cc = 0; cc < NCH; ++cc)
           for (int bx = 0; bx < NBOX; ++bx) {
@@ -270,7 +271,7 @@ __global__ void __launch_bounds__(RB_THREADS, 1) tc_rbstep_kernel(const __grid_c
         // ---------------- E1(it): a1 = lrelu(conv1 + b1) -> shared-memory A tiles of conv2 ----------------
         const int tile = (int)blockIdx.x + it * (int)gridDim.x;
         const int tt = tile % p.t_tiles, b = tile / p.t_tiles;
-        const int t = tt * R_OUT - h2 + m;                     // time step of this a1 row
+        const int t = p.row0 + tt * R_OUT - h2 + m;                     // time step of this a1 row
         const int len = p.lens ? min(p.lens[b], p.L) : p.L;
         const bool valid = t >= 0 && t < len;                  // outside the utterance a1 is the conv's ZERO padding
         mbar_wait(a1full, it & 1);
@@ -333,7 +334,7 @@ __global__ void __launch_bounds__(RB_THREADS, 1) tc_rbstep_kernel(const __grid_c
         const int jt = it - 1;
         const int tile = (int)blockIdx.x + jt * (int)gridDim.x;
         const int tt = tile % p.t_tiles, b = tile / p.t_tiles;
-        const int t = tt * R_OUT + m;
+        const int t = p.row0 + tt * R_OUT + m;
         const int len = p.lens ? min(p.lens[b], p.L) : p.L;
         const bool o_in = m < R_OUT && t < p.L;                // rows this tile owns
         const bool o_valid = o_in && t < len;

@@ -9,12 +9,13 @@ cube/networks/cubegan.py:83, cube/io_utils/runtime.py:51-54,78).  Inference only
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, Mapping, Optional, Sequence
+from typing import Dict, List, Mapping, Optional, Sequence, Tuple
 
 import torch
 
 from . import _lib
 from ._lib import VocConfig, check, lib
+from .streaming import HifiganStream, step_streams
 
 
 def _cfg_get(h, key, default=None):
@@ -78,6 +79,39 @@ class _Handle:
                 C.c_void_p(wav.data_ptr()), C.c_void_p(w16.data_ptr()) if w16 is not None else None,
                 B, F, C.c_void_p(_stream_ptr(mel.device))))
         return (wav, w16) if want_int16 else wav
+
+    def forward_range(self, mel: torch.Tensor, n_frames: Optional[Sequence[int]], begin: Sequence[int],
+                      end: Sequence[int], want_int16: bool = False, out: Optional[torch.Tensor] = None):
+        """cube_voc_forward_range: only samples [begin[b], end[b]) of item b are written (into `out`, [B, 1, T] float32
+        or [B, T] int16, when given).  Returns (out, list of the B requested slices)."""
+        if mel.device.type != "cuda" or mel.dtype != torch.float32 or mel.dim() != 3:
+            raise _lib.CubeVocError(f"mel must be float32 [B, C, F] on a CUDA device, got {mel.dtype} {tuple(mel.shape)} on {mel.device}")
+        self._check_shapes(mel, n_frames)
+        if mel.device != self.device:
+            raise _lib.CubeVocError(f"mel lives on {mel.device} but this vocoder's weights live on {self.device}")
+        mel = mel.contiguous()
+        B, _, F = mel.shape
+        if len(begin) != B or len(end) != B:
+            raise _lib.CubeVocError(f"begin / end need {B} entries, got {len(begin)} / {len(end)}")
+        T = self.out_len(F)
+        shape, dt = ((B, T), torch.int16) if want_int16 else ((B, 1, T), torch.float32)
+        if out is None:
+            out = torch.empty(*shape, device=mel.device, dtype=dt)
+        elif tuple(out.shape) != shape or out.dtype != dt or out.device != mel.device or not out.is_contiguous():
+            raise _lib.CubeVocError(f"`out` must be a contiguous {dt} {shape} tensor on {mel.device}")
+        nf = (C.c_int32 * B)(*[int(v) for v in n_frames]) if n_frames is not None else None
+        b0 = (C.c_int64 * B)(*[int(v) for v in begin])
+        b1 = (C.c_int64 * B)(*[int(v) for v in end])
+        wav = None
+        if want_int16:   # the float32 samples go to a scratch tensor the caller never sees
+            wav = torch.empty(B, 1, T, device=mel.device, dtype=torch.float32)
+        with torch.cuda.device(mel.device):
+            check(lib().cube_voc_forward_range(
+                self.ptr, C.c_void_p(mel.data_ptr()), nf, b0, b1,
+                C.c_void_p((wav if want_int16 else out).data_ptr()), C.c_void_p(out.data_ptr()) if want_int16 else None,
+                B, F, C.c_void_p(_stream_ptr(mel.device))))
+        flat = out.view(B, T)
+        return out, [flat[b, int(begin[b]):int(end[b])] for b in range(B)]
 
     def _check_shapes(self, mel: torch.Tensor, n_frames) -> None:
         """The engine trusts num_mels and B: a narrower tensor or a short n_frames list would be read out of bounds."""
@@ -254,6 +288,44 @@ class CubeGenerator(torch.nn.Module):
     def forward_int16(self, x: torch.Tensor, n_frames: Optional[Sequence[int]] = None):
         """Fused cube/api.py:64-65 epilogue: returns (wav float32 [B,1,T], int16 [B,T])."""
         return self._ensure().forward(x, n_frames, None, want_int16=True)
+
+    # ---- streaming (tts_cube_b200/streaming.py) ------------------------------------------------
+    @property
+    def hop(self) -> int:
+        """Output samples per mel frame: prod(upsample_rates)."""
+        n = 1
+        for i in range(self._cfg.n_ups):
+            n *= int(self._cfg.upsample_rates[i])
+        return n
+
+    def sample_support(self, s0: int, s1: int) -> Tuple[int, int]:
+        """Mel frames [f0, f1) that output samples [s0, s1) depend on (f0 clipped at 0, f1 not clipped).  No GPU needed."""
+        f0, f1 = C.c_int64(), C.c_int64()
+        check(lib().cube_voc_hifigan_support(C.byref(self._cfg), int(s0), int(s1), C.byref(f0), C.byref(f1)))
+        return int(f0.value), int(f1.value)
+
+    def forward_range(self, mel: torch.Tensor, n_frames: Optional[Sequence[int]], begin: Sequence[int],
+                      end: Sequence[int], int16: bool = False, out: Optional[torch.Tensor] = None) -> List[torch.Tensor]:
+        """Samples [begin[b], end[b]) of generator(mel[b, :, :n_frames[b]]), bit-identical to forward(); one tensor of
+        end[b] - begin[b] samples per item (views into `out` when given: [B, 1, T] float32 or [B, T] int16, whose other
+        elements are left untouched)."""
+        return self._ensure().forward_range(mel, n_frames, begin, end, want_int16=int16, out=out)[1]
+
+    def open_stream(self, int16: bool = False) -> HifiganStream:
+        """A session fed mel chunks [num_mels, f]; see HifiganStream."""
+        return HifiganStream(self.sample_support, self.out_len, self.hop, int(self._cfg.num_mels), int16=int16, owner=self)
+
+    def step_streams(self, streams: Sequence[HifiganStream]) -> List[torch.Tensor]:
+        """One batched forward_range over the sessions (one per output type) -> each session's newly final samples."""
+        out: List[Optional[torch.Tensor]] = [None] * len(streams)
+        for i16 in (False, True):
+            idx = [i for i, s in enumerate(streams) if s.int16 == i16]
+            if not idx:
+                continue
+            vr = lambda m, nf, b, e, i16=i16: self.forward_range(m, nf, b, e, int16=i16)  # noqa: E731
+            for i, piece in zip(idx, step_streams([streams[i] for i in idx], vr, device=self.device)):
+                out[i] = piece
+        return out  # type: ignore
 
     def forward_host(self, mel: torch.Tensor, n_frames=None, out: Optional[torch.Tensor] = None,
                      int16: bool = False) -> torch.Tensor:
